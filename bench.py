@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W                      # N GPUs, one rank each (data parallel, NCCL)
     python bench.py --impl reference --steps 2 --warmup 1              # the reference algorithm on the host CPU cores
+    python bench.py --steps 20 --warmup 5 --dump-outputs DIR          # also writes the last timed step's outputs as DIR/*.npy
 
 A step = one full training step of 4M-B mod7 (BASELINE.json configs[1]): forward + backward + gradient all-reduce (DDP)
 + AdamW, per-GPU batch 128, 128 encoder + 128 decoder tokens per sample, synthetic data, random-init weights.
@@ -279,6 +280,22 @@ def run_reference_arm(args):
 # ----------------------------------------------------------------------------------------------------------------------
 # B200 arm
 # ----------------------------------------------------------------------------------------------------------------------
+PARAM_SAMPLE = 1 << 21          # parameter values written by --dump-outputs (8 MB of float32)
+
+
+def dump_outputs(out_dir, loss, mod_loss, gnorm, model):
+    """Writes what one train step returns (loss, per-modality losses, gradient norm) and a fixed, seeded sample of the parameters it
+    updated to out_dir/<name>.npy as float32, so that two builds run with the same arguments can be compared array by array."""
+    import numpy as np
+    arrays = {"loss": loss, "grad_norm": gnorm, **{f"mod_loss.{m}": v for m, v in mod_loss.items()}}
+    flat = torch.cat([p.detach().reshape(-1).float() for p in model.parameters()])
+    idx = torch.randint(0, flat.numel(), (min(PARAM_SAMPLE, flat.numel()),), generator=torch.Generator().manual_seed(0)).sort().values
+    arrays["params_sample"] = flat[idx.to(flat.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def run_b200_arm(args):
     import torch.distributed as dist
     from b200fm import lib, ops
@@ -405,6 +422,7 @@ def run_b200_arm(args):
         n_calls = lib.CALLS["n"] - calls0
         if gstep is not None and gstep.graph is not None:
             n_calls += gstep.kernel_calls_per_step * n_steps        # launches replayed from the captured graph
+        timed.outputs = (loss, mod_loss, gnorm)                      # the last step's results, valid until the next step
         return ms, n_calls, (last if last is not None else float(loss.item()))
 
     for _ in range(max(args.warmup, 3)):
@@ -421,6 +439,8 @@ def run_b200_arm(args):
         sampler.start()
     ms, launches, loss_val = timed(args.steps, e2e=False)
     cpu_issue_ms = timed.cpu_ms
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *timed.outputs, model)
     # end to end.  Wire format of the RGB modality: "uint8" (default) ships the raw 8-bit pixels and applies the loader's ToTensor +
     # Normalize inside the patchify kernel (fourm/models/encoder_embeddings.py, b200fm.masking): 22 MB per step over PCIe instead of the
     # 80 MB of the reference's fp32 wire format, which is measured as well (`e2e_fp32_wire`).  Same step otherwise.
@@ -865,7 +885,12 @@ def main():
     ap.add_argument("--batch", type=int, default=None, help="per-GPU batch (default: the workload's reference config)")
     ap.add_argument("--tokens", type=int, default=None, help="encoder tokens = decoder tokens per sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's loss, per-modality losses, gradient norm and a seeded parameter sample as "
+                         "DIR/<name>.npy (4m-b / 4m-l on the GPU)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload not in WORKLOADS):
+        ap.error("--dump-outputs is implemented for the GPU train step (--workload 4m-b / 4m-l)")
     if args.impl == "reference":
         run_reference_arm(args)
     elif args.workload in ("vq-tokenize", "vqvae-train"):

@@ -134,9 +134,39 @@ def main():
                   sincos2d_14x14x384_sum=fm_utils.build_2d_sincos_posemb(14, 14, 384).double().sum(-1))
     torch.save(static, os.path.join(HERE, "static_golden.pt"))
 
-    # ---- VQ tokenizer forward (a20-a24) ----
+    # ---- VQ tokenizer forward (a20-a24): in a subprocess under REPRODUCIBLE_CPU_ENV, like the test that compares against it ----
+    import subprocess
+    import tempfile
+    from tests.helpers import REPRODUCIBLE_CPU_ENV
+    with tempfile.TemporaryDirectory() as tmp:
+        subprocess.run([sys.executable, os.path.abspath(__file__), "vq_encode_cases", os.path.join(tmp, "cases.pt")], check=True,
+                       env={**os.environ, **REPRODUCIBLE_CPU_ENV})
+        vgold = dict(meta=meta, cases=torch.load(os.path.join(tmp, "cases.pt"), weights_only=False))
+    import fourm.vq as vq  # noqa: F401
+    # stand-alone codebook scan KATs (a23/a24) straight through the reference codebook classes
+    from fourm.vq.quantizers.quantize_lucid import CosineSimCodebook, EuclideanCodebook
+    g = torch.Generator().manual_seed(11)
+    z = torch.randn(1, 777, 32, generator=g)
+    cb = CosineSimCodebook(dim=32, codebook_size=2048).eval()
+    cb.embed.copy_(torch.nn.functional.normalize(torch.randn(2048, 32, generator=g), dim=-1))
+    eb = EuclideanCodebook(dim=32, codebook_size=1000).eval()
+    eb.embed.copy_(torch.randn(1000, 32, generator=g))
+    with torch.no_grad():
+        qc, ic = cb(z)
+        qe, ie = eb(z)
+    vgold["scan"] = dict(z=z[0].clone(), cos_embed=cb.embed.clone(), cos_idx=ic[0].clone(), cos_quant=qc[0].clone(),
+                         l2_embed=eb.embed.clone(), l2_idx=ie[0].clone(), l2_quant=qe[0].clone())
+    torch.save(vgold, os.path.join(HERE, "vq_golden.pt"))
+    for f in ("fourm_tiny_golden.pt", "static_golden.pt", "vq_golden.pt"):
+        print(f, os.path.getsize(os.path.join(HERE, f)) // 1024, "KiB")
+
+
+def vq_encode_cases():
+    """VQ.encode of the reference tokenizer on deterministic weights, for the two tokenizer cases of vq_golden.pt."""
+    torch.set_num_threads(1)
+    ref_import.install()
     import fourm.vq as vq
-    vgold = dict(meta=meta, cases={})
+    cases = {}
     for tag, kw in {
         "vit_s_cos": dict(enc_type="vit_s_enc", image_size=64, codebook_size=1024, latent_dim=32, norm_codes=True, post_mlp=True),
         "vit_s_l2": dict(enc_type="vit_s_enc", image_size=64, codebook_size=512, latent_dim=32, norm_codes=False, post_mlp=False),
@@ -157,27 +187,15 @@ def main():
         with torch.no_grad():
             quant, code_loss, tokens = m.encode(x)
             h = m.quant_proj(m.encoder(x))
-        vgold["cases"][tag] = dict(kw=kw, shapes={k: tuple(v.shape) for k, v in vsd.items()},
-                                   weight_checksums={k: float(v.double().sum()) for k, v in vsd.items()},
-                                   tokens=tokens.clone(), latents=h.clone(), quant=quant.clone())
+        cases[tag] = dict(kw=kw, shapes={k: tuple(v.shape) for k, v in vsd.items()},
+                          weight_checksums={k: float(v.double().sum()) for k, v in vsd.items()},
+                          tokens=tokens.clone(), latents=h.clone(), quant=quant.clone())
         print(tag, tokens.flatten()[:8].tolist())
-    # stand-alone codebook scan KATs (a23/a24) straight through the reference codebook classes
-    from fourm.vq.quantizers.quantize_lucid import CosineSimCodebook, EuclideanCodebook
-    g = torch.Generator().manual_seed(11)
-    z = torch.randn(1, 777, 32, generator=g)
-    cb = CosineSimCodebook(dim=32, codebook_size=2048).eval()
-    cb.embed.copy_(torch.nn.functional.normalize(torch.randn(2048, 32, generator=g), dim=-1))
-    eb = EuclideanCodebook(dim=32, codebook_size=1000).eval()
-    eb.embed.copy_(torch.randn(1000, 32, generator=g))
-    with torch.no_grad():
-        qc, ic = cb(z)
-        qe, ie = eb(z)
-    vgold["scan"] = dict(z=z[0].clone(), cos_embed=cb.embed.clone(), cos_idx=ic[0].clone(), cos_quant=qc[0].clone(),
-                         l2_embed=eb.embed.clone(), l2_idx=ie[0].clone(), l2_quant=qe[0].clone())
-    torch.save(vgold, os.path.join(HERE, "vq_golden.pt"))
-    for f in ("fourm_tiny_golden.pt", "static_golden.pt", "vq_golden.pt"):
-        print(f, os.path.getsize(os.path.join(HERE, f)) // 1024, "KiB")
+    return cases
 
 
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:2] == ["vq_encode_cases"]:
+        torch.save(vq_encode_cases(), sys.argv[2])
+    else:
+        main()

@@ -11,6 +11,12 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 GOLDEN = os.path.join(HERE, "golden")
 
+# fp32 CPU results that do not depend on the host: MKL's reproducible code path, ATen and oneDNN kernels at the baseline ISA, one
+# thread.  Deep fp32 networks otherwise differ by more than their tolerance between BLAS code paths and thread counts.  MKL reads
+# these at start-up, so a computation that needs them runs in a subprocess with this environment.
+REPRODUCIBLE_CPU_ENV = dict(MKL_CBWR="COMPATIBLE", ATEN_CPU_CAPABILITY="default", ONEDNN_MAX_CPU_ISA="SSE41", OMP_NUM_THREADS="1",
+                            MKL_NUM_THREADS="1")
+
 
 def load_golden(name):
     return torch.load(os.path.join(GOLDEN, name), weights_only=False)

@@ -67,10 +67,12 @@ def test_library_is_tcgen05_tma_code(built):
     import re
     import shutil
     import subprocess
-    if shutil.which("cuobjdump") is None:
-        pytest.skip("cuobjdump not on PATH")
-    from b200fm import lib
-    sass = subprocess.run(["cuobjdump", "-sass", lib.LIB_PATH], capture_output=True, text=True, timeout=600).stdout
+    from b200fm import build, lib
+    # the toolkit that built the library ships cuobjdump next to nvcc, whether or not it is on PATH
+    cuobjdump = shutil.which("cuobjdump", path=os.path.dirname(build.NVCC)) or shutil.which("cuobjdump")
+    if cuobjdump is None:
+        pytest.skip("cuobjdump not found")
+    sass = subprocess.run([cuobjdump, "-sass", lib.LIB_PATH], capture_output=True, text=True, timeout=600).stdout
     assert "sm_100a" in sass or "SM100" in sass.upper()
     per_fn, cur = {}, None
     for line in sass.splitlines():

@@ -239,33 +239,82 @@ def test_tokenizer_constructors_match_reference_state_dict_contract():
         assert mgp.digest(m) == gold[tag], (tag, mgp.digest(m), gold[tag])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/fourm"), reason="needs the reference tree (authoring container only)")
-def test_overlay_resolves_ahead_of_reference_tree():
+# the parts of the reference the overlay talks to, restated minimally for the stand-in tree: the timm-style model registry and the
+# `create_model` that looks names up in it, and MODALITY_INFO rebuilt from the recorded embedding factories
+_STANDIN = {
+    "fourm/utils/timm/registry.py": '''
+_model_entrypoints = {{}}
+
+
+def register_model(fn):
+    _model_entrypoints[fn.__name__] = fn
+    return fn
+
+
+def model_entrypoint(model_name):
+    return _model_entrypoints[model_name]
+''',
+    "fourm/utils/__init__.py": '''
+from .timm.registry import model_entrypoint, register_model
+
+
+def create_model(model_name, **kwargs):
+    return model_entrypoint(model_name)(**kwargs)
+''',
+    "fourm/data/modality_info.py": '''
+import importlib
+import json
+from functools import partial
+
+with open({golden!r}) as f:
+    _entries = json.load(f)["modality_info"]
+
+
+def _factory(spec):
+    return None if spec is None else partial(getattr(importlib.import_module(spec["module"]), spec["name"]), **spec["kwargs"])
+
+
+MODALITY_INFO = {{m: {{k: _factory(v) if k.endswith("_embedding") else v for k, v in e.items()}} for m, e in _entries.items()}}
+''',
+}
+
+
+def test_overlay_resolves_ahead_of_reference_tree(tmp_path):
     """INTEGRATION.md level 1: with `ml-4m_b200/` ahead of the reference on sys.path, exactly the hot-path modules resolve to the overlay
-    (fourm.models.fm / fm_utils / *_embeddings, fourm.vq) while fourm.utils, fourm.data and fourm.models.generate stay the reference's;
-    the reference's own `create_model` + `MODALITY_INFO` factories then build the overlay classes and `GenerationSampler` wraps them."""
+    (fourm.models.fm / fm_utils / *_embeddings / generate, fourm.vq) while fourm.utils and fourm.data stay the reference's; the
+    reference's registry-based `create_model` + `MODALITY_INFO` factories then build the overlay classes and `GenerationSampler` wraps
+    them.  The reference is a stand-in tree with the unmodified reference's package layout (every module empty except the registry,
+    `create_model` and MODALITY_INFO); the layout, the resolution and the built class were recorded from the unmodified reference
+    (fixture: tests/golden/make_golden_overlay.py)."""
+    golden_path = os.path.join(ROOT, "tests", "golden", "overlay_golden.json")
+    gold = json.load(open(golden_path))
+    ref = tmp_path / "reference"
+    for rel in gold["layout"]:
+        (ref / rel).parent.mkdir(parents=True, exist_ok=True)
+        (ref / rel).write_text(_STANDIN.get(rel, "").format(golden=golden_path))
+    assert set(_STANDIN) <= set(gold["layout"])
     code = r'''
-import sys
-sys.path.insert(0, "{root}/tests/golden")
-import ref_import
-ref_import.install(extra_first_paths=["{root}/ml-4m_b200"])
-import fourm.models.fm as fm, fourm.models.fm_utils as fu, fourm.models.encoder_embeddings as ee, fourm.vq as vq
+import json, sys
+ov, ref = {ov!r}, {ref!r}
+sys.path[:0] = [ov, ref]
+gold = json.load(open({golden!r}))
+import importlib
+where = lambda f: "overlay" if f.startswith(ov + "/") else "reference" if f.startswith(ref + "/") else f
+assert {{m: where(importlib.import_module(m).__file__) for m in gold["resolved"]}} == gold["resolved"]
 import fourm.utils as utils, fourm.models.generate as gen
 from fourm.data.modality_info import MODALITY_INFO
-ov, ref = "{root}/ml-4m_b200/", "/root/reference/"
-assert fm.__file__.startswith(ov) and fu.__file__.startswith(ov) and ee.__file__.startswith(ov) and vq.__file__.startswith(ov)
-assert utils.__file__.startswith(ref) and gen.__file__.startswith(ov)      # generation is an overlay module since round 2
-mods = ["rgb@224", "caption", "tok_depth@224"]
+mods = list(gold["modality_info"])
 mk = lambda m, side: MODALITY_INFO[m][side]() if MODALITY_INFO[m]["type"] != "img" else MODALITY_INFO[m][side](patch_size=16, image_size=224)
 enc = {{m: mk(m, "encoder_embedding") for m in mods}}
 dec = {{m: mk(m, "decoder_embedding") for m in mods[1:]}}
 model = utils.create_model("fm_tiny_6e_6d_swiglu_nobias", encoder_embeddings=enc, decoder_embeddings=dec, modality_info={{m: MODALITY_INFO[m] for m in mods}})
-assert type(model).__module__ == "fourm.models.fm" and sys.modules["fourm.models.fm"].__file__.startswith(ov)
+assert [type(model).__module__, type(model).__name__] == gold["model_class"]
+assert where(sys.modules[type(model).__module__].__file__) == "overlay"
 assert hasattr(model.encoder[0], "forward_pending")            # the overlay's block, not the reference's
 gen.GenerationSampler(model)
 print("OK")
-'''.format(root=ROOT)
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300, cwd="/tmp",
+'''.format(ov=os.path.join(ROOT, "ml-4m_b200"), ref=str(ref), golden=golden_path)
+    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300, cwd=tmp_path,
                          env={**os.environ, "PYTHONPATH": ""})
     assert out.returncode == 0 and "OK" in out.stdout, out.stderr[-2000:]
 

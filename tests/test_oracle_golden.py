@@ -1,4 +1,8 @@
 """The oracle restatement vs. the golden outputs of the UNMODIFIED reference (CPU, no GPU)."""
+import os
+import subprocess
+import sys
+
 import torch
 import pytest
 
@@ -107,10 +111,10 @@ def test_fully_masked_row_is_uniform():
     torch.testing.assert_close(out[0, 0, 0], v[0, 0].mean(0))
 
 
-@pytest.mark.parametrize("tag", ["vit_s_cos", "vit_s_l2"])
-def test_vq_encode_matches_reference(tag):
-    gold = H.load_golden("vq_golden.pt")
-    c = gold["cases"][tag]
+def _vq_encode_case(tag, out):
+    """The oracle's VQ.encode of a golden case on the fixture weights -> torch.save((quant, tokens, latents), out)."""
+    torch.set_num_threads(1)
+    c = H.load_golden("vq_golden.pt")["cases"][tag]
     kw = c["kw"]
     sd = {}
     for k, shape in c["shapes"].items():
@@ -128,7 +132,19 @@ def test_vq_encode_matches_reference(tag):
             sd[k] = O.deterministic_tensor(k, shape, 0.05 if len(shape) > 1 else 0.02)
         assert abs(float(sd[k].double().sum()) - c["weight_checksums"][k]) <= 1e-5 * max(1.0, abs(c["weight_checksums"][k])), k
     x = torch.randn(3, 3, 64, 64, generator=torch.Generator().manual_seed(5))
-    quant, tokens, lat = V.vq_encode(x, sd, kw["enc_type"], 16, kw["norm_codes"], kw["post_mlp"])
+    torch.save(V.vq_encode(x, sd, kw["enc_type"], 16, kw["norm_codes"], kw["post_mlp"]), out)
+
+
+@pytest.mark.parametrize("tag", ["vit_s_cos", "vit_s_l2"])
+def test_vq_encode_matches_reference(tag, tmp_path):
+    """Both sides run in fp32 under helpers.REPRODUCIBLE_CPU_ENV (the reference's: make_golden.py), so the comparison does not depend
+    on the host's BLAS code path or thread count."""
+    c = H.load_golden("vq_golden.pt")["cases"][tag]
+    out = tmp_path / "vq_encode.pt"
+    subprocess.run([sys.executable, "-c", f"from tests.test_oracle_golden import _vq_encode_case; _vq_encode_case({tag!r}, {str(out)!r})"],
+                   cwd=H.ROOT, env={**os.environ, **H.REPRODUCIBLE_CPU_ENV, "PYTHONPATH": os.pathsep.join([H.ROOT, os.path.join(H.ROOT, "ml-4m_b200")])},
+                   check=True)
+    quant, tokens, lat = torch.load(out)
     torch.testing.assert_close(lat, c["latents"], rtol=1e-4, atol=1e-5)
     assert torch.equal(tokens, c["tokens"])
     torch.testing.assert_close(quant, c["quant"])
